@@ -4,6 +4,7 @@ base_with_context, 1000-step DDPM).
 
   python bench.py --gpus N --steps K --warmup W        # this repo's sm_100a path
   python bench.py --impl reference ...                 # the CPU oracle port on the host cores
+  python bench.py ... --dump-outputs DIR               # + the last timed step's mel in DIR/mel.npy
 
 A "step" is one pass of the hot path over one batch: `predict` of `--segments` independent
 5.12 s segments per GPU (encode + num_steps reverse-diffusion steps + unscale).  Under torchrun
@@ -407,6 +408,23 @@ def measure_gemm_traffic(args, timeout_s=240):
                  'launches of one uncaptured diffusion step, measured in this run'}
 
 
+DUMP_BUDGET_BYTES = 60_000_000  # under 64 MB (decimal or binary) with the .npy headers and index file
+
+
+def dump_outputs(directory, name, mel, budget=DUMP_BUDGET_BYTES):
+  """Writes `mel` [segments, frames, n_dims] as <directory>/<name>.npy (float32), so that two
+  builds can be compared output for output.  Past `budget` bytes it writes a fixed seeded sample
+  of whole segments instead, and their indices as <name>_segments.npy."""
+  mel = mel.float().cpu().numpy()
+  os.makedirs(directory, exist_ok=True)
+  keep = budget // (mel[0].nbytes + 8)
+  if mel.shape[0] > keep:
+    idx = np.sort(np.random.default_rng(0).choice(mel.shape[0], keep, replace=False))
+    mel = mel[idx]
+    np.save(os.path.join(directory, f'{name}_segments.npy'), idx.astype(np.float64))
+  np.save(os.path.join(directory, f'{name}.npy'), mel)
+
+
 def synthetic_song_notes(segments, lengths):
   """A multi-instrument synthetic arrangement covering `segments` 5.12 s segments."""
   from music_spectrogram_diffusion_b200 import midi_tokens
@@ -538,6 +556,9 @@ def run_ours(args):
     return float(t.item()) / 1e3, wall, clocks, eng_mod.launch_count() - launches0
 
   sec, wall, clocks, launches = timed(device_step, args.warmup, args.steps)
+  if args.dump_outputs:
+    dump_outputs(args.dump_outputs, 'mel' if world == 1 else f'mel_rank{rank}', d_mel,
+                 DUMP_BUDGET_BYTES // world)
   frames = world * B * lengths['targets'] * args.steps
   value = frames / sec
   sec_e2e, wall_e2e, clocks_e2e, _ = timed(host_step, max(1, args.warmup // 2), args.steps)
@@ -674,7 +695,14 @@ def main():
                   help='skip the batch-1 chained-song sample (BASELINE config 5)')
   ap.add_argument('--song-segments', type=int, default=12,
                   help='segments of the chained song (12 = 61.44 s, BASELINE config 5)')
+  ap.add_argument('--dump-outputs', metavar='DIR',
+                  help='after the timed steps, write the mel batch of the last one as DIR/mel.npy '
+                       '(DIR/mel_rank<r>.npy per rank under torchrun)')
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
+  if args.dump_outputs and args.impl != 'ours':
+    ap.error('--dump-outputs writes the outputs of --impl ours')
   if args.impl == 'reference':
     run_reference(args)
   else:

@@ -15,11 +15,11 @@ from oracle import msd_oracle as O  # noqa: E402
 from tests import helpers as H  # noqa: E402
 
 T = N = C = 128
-STEPS, W, B = 12, 2.0, 2
+STEPS, W, B, NOISE_SEED = 12, 2.0, 2, 0
 t5 = config.t5_tiny()
 params = weights.synthetic_params(t5, T, N, C, seed=0)
 toks, ctx, cmask = H.make_batch(B, T, C)
-init_z, noise = H.make_noise(STEPS, B, N)
+init_z, noise = H.make_noise(STEPS, B, N, seed=NOISE_SEED)
 oc = H.oracle_config(t5, STEPS, W)
 P = O.params_to(params)
 batch = H.torch_batch(toks, ctx, cmask)
@@ -28,8 +28,10 @@ encs = O.encode(P, oc, batch['encoder_input_tokens'],
                 O.scale_features(batch['encoder_continuous_inputs'], oc, clip=True),
                 batch['encoder_continuous_mask'])
 eps_first = O.decode(P, oc, encs, init_z, torch.full((B,), 1.0))
+# the noise itself is redrawn from NOISE_SEED by tests/helpers.tiny_golden; a sample pins it
 np.savez_compressed(
     os.path.join(os.path.dirname(os.path.abspath(__file__)), 'tiny_predict.npz'),
-    tokens=toks, ctx=ctx, ctx_mask=cmask, init_z=init_z.numpy(), noise=noise.numpy(),
-    mel=mel.numpy(), eps_first=eps_first.numpy(), steps=STEPS, cond_weight=W)
+    tokens=toks, ctx=ctx, ctx_mask=cmask, init_z=init_z.numpy(), noise_seed=NOISE_SEED,
+    noise_sample=noise[:, :, 0, :8].numpy(), mel=mel.numpy(), eps_first=eps_first.numpy(),
+    steps=STEPS, cond_weight=W)
 print('wrote tiny_predict.npz', mel.shape, float(mel.mean()))

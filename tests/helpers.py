@@ -39,6 +39,19 @@ def make_noise(steps, B, N, seed=0):
   return init_z, noise
 
 
+def tiny_golden(path):
+  """tests/golden/tiny_predict.npz (tests/golden/make_golden.py) as a dict.  The per-step noise
+  (1.6 MB of incompressible floats) is not stored: it is redrawn by make_noise from the stored
+  seed, and the stored init_z and noise sample fail the load if that stream ever changes."""
+  g = dict(np.load(path))
+  init_z, noise = make_noise(int(g['steps']), g['init_z'].shape[0], g['init_z'].shape[1],
+                             seed=int(g['noise_seed']))
+  np.testing.assert_array_equal(init_z.numpy(), g['init_z'])
+  np.testing.assert_array_equal(noise[:, :, 0, :8].numpy(), g['noise_sample'])
+  g['noise'] = noise.numpy()
+  return g
+
+
 def build_engine(t5, T, N, C, B, steps, cond_weight, params, sampler='ddpm', logvar='large',
                  clip_x0=True, model_output='eps', schedule=None, train_schedule=None,
                  precision='bf16'):

@@ -384,7 +384,7 @@ def test_inference_model_predict_matches_golden_fixture(cuda_device):
   fixture tests/golden/tiny_predict.npz (oracle outputs, see make_golden.py)."""
   import os
   from music_spectrogram_diffusion_b200 import inference
-  g = np.load(os.path.join(os.path.dirname(__file__), 'golden', 'tiny_predict.npz'))
+  g = H.tiny_golden(os.path.join(os.path.dirname(__file__), 'golden', 'tiny_predict.npz'))
   t5 = config.t5_tiny()
   diff = config.DiffusionConfig()
   diff.sampler.schedule.num_steps = int(g['steps'])

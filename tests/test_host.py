@@ -203,24 +203,45 @@ def test_gin_bindings_reach_the_sampler_variants():
   assert abs(cfg.sampler_beta_start - 1e-4) < 1e-9 and abs(cfg.sampler_beta_stop - 0.02) < 1e-8
 
 
-REF_GIN = '/root/reference/music_spectrogram_diffusion/gin'
+GIN_INCLUDE_ROOT = os.path.join(HERE, 'golden', 'gin_include')
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_GIN), reason='reference tree not present on this box')
-def test_every_reference_gin_file_parses():
-  """gin_lite reads the subset of gin the reference's config files use (includes, macros,
-  scoped bindings, configurable references, multi-line values)."""
-  import glob
-  files = sorted(glob.glob(os.path.join(REF_GIN, '**', '*.gin'), recursive=True))
-  assert len(files) >= 25
-  for f in files:
-    gin_lite.parse_config(open(f).read(), ['/root/reference'])
-  sizes = {}
-  for name in ('local_tiny', 't5_small', 't5_base', 't5_large'):
-    g = gin_lite.parse_config(open(os.path.join(REF_GIN, 'models/diffusion/context', name + '.gin')).read(),
-                              ['/root/reference'])
-    b = g.bindings_for('network.T5Config')
-    sizes[name] = (b['emb_dim'], b['num_heads'], b['num_decoder_layers'], b['mlp_dim'])
+def test_gin_lite_includes_across_files():
+  """gin_lite reads the subset of gin the reference's config files use: nested includes resolved
+  against a search root, macros (resolved when queried), scoped bindings, configurable references,
+  bracket and backslash continuations, and later bindings overriding included ones."""
+  with open(os.path.join(GIN_INCLUDE_ROOT, 'configs', 'model.gin')) as f:
+    g = gin_lite.parse_config(f.read(), [GIN_INCLUDE_ROOT])
+  assert g.query_macro('TASK_FEATURE_LENGTHS') == {'inputs': 2048, 'targets': 256,
+                                                   'targets_context': 256}
+  assert g.query_macro('NUM_VELOCITY_BINS') == 1
+  assert g.query_macro('%DECODER_LAYERS') == 8
+  codec, model = g.macros['AUDIO_CODEC'], g.macros['MODEL']
+  assert isinstance(codec, gin_lite.ConfigurableRef) and codec.evaluate
+  assert (codec.scope, codec.name) == ('', 'audio_codecs.MelGAN')
+  assert model.name == 'models.ContextDiffusionModel'
+  t5 = g.bindings_for('network.T5Config')
+  assert t5['emb_dim'] == 512 and g.resolve(t5['num_decoder_layers']) == 8
+  assert t5['mlp_activations'] == ('gelu', 'linear')
+  assert t5['dropout_rate'] == 0.0
+  assert isinstance(t5['vocab_size'], gin_lite.ConfigurableRef) and t5['vocab_size'].evaluate
+  assert g.bindings_for('diffusion_utils.DiffusionSchedule', 'train') == {'name': 'linear'}
+  assert g.bindings_for('diffusion_utils.DiffusionSchedule', 'sampler') == {'name': 'cosine',
+                                                                          'num_steps': 250}
+  assert g.bindings_for('diffusion_utils.DiffusionSchedule') == {'name': 'cosine'}
+  with pytest.raises(FileNotFoundError):
+    gin_lite.parse_config("include 'configs/missing.gin'", [GIN_INCLUDE_ROOT])
+
+
+def test_reference_model_sizes_match_config():
+  """The network.T5Config sizes gin_lite reads from the reference's
+  gin/models/diffusion/context/*.gin (stored by tests/golden/make_reference_gin_sizes.py) are the
+  ones config.py builds."""
+  import json
+  with open(os.path.join(HERE, 'golden', 'reference_gin_model_sizes.json')) as f:
+    sizes = {name: (s['emb_dim'], s['num_heads'], s['num_decoder_layers'], s['mlp_dim'])
+             for name, s in json.load(f).items()}
+  assert set(sizes) == {'local_tiny', 't5_small', 't5_base', 't5_large'}
   base, small = config.t5_base(), config.t5_small()
   assert sizes['t5_base'] == (base.emb_dim, base.num_heads, base.num_decoder_layers, base.mlp_dim)
   assert sizes['t5_small'] == (small.emb_dim, small.num_heads, small.num_decoder_layers, small.mlp_dim)

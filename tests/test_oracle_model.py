@@ -121,7 +121,7 @@ def test_golden_fixture_matches_live_oracle(tiny):
   """tests/golden/tiny_predict.npz (written by tests/golden/make_golden.py) pins today's oracle
   output so an accidental change of the restatement is caught."""
   t5, params = tiny
-  g = np.load(GOLDEN)
+  g = H.tiny_golden(GOLDEN)
   steps = int(g['steps'])
   oc = H.oracle_config(t5, steps, float(g['cond_weight']))
   batch = dict(encoder_input_tokens=torch.from_numpy(g['tokens']),
